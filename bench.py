@@ -2,6 +2,7 @@
 """bench.py -- KVStore push+pull throughput on the ResNet-50 gradient set (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload ...]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the synthetic gradient set: push the gradients of all
 157 ResNet-50 tensors (25 549 486 fp32 elements, uniform [-1,1)), reduce them, apply SGD with
@@ -468,6 +469,36 @@ def per_key_step_fns(mx, kv, keys, vals, outs):
     return issue(0), issue(1), python_loop
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_SEED = 0xB200 + 31
+
+
+def dump_outputs(dump_dir, arrays):
+    """Write what the last timed step handed its caller as DIR/<name>.npy, flattened; `arrays` maps
+    names to float32 / float64 numpy arrays. Every file keeps at most the byte count that keeps them
+    all under DUMP_LIMIT_BYTES; a longer array is written as the values at sorted positions drawn by
+    np.random.default_rng(DUMP_SAMPLE_SEED + its index in `arrays`), so the files of two builds run
+    with the same arguments compare value for value."""
+    arrays = [(name, np.ascontiguousarray(a).reshape(-1)) for name, a in arrays.items()]
+    sizes = sorted(a.nbytes for _, a in arrays)
+    budget, cap = DUMP_LIMIT_BYTES - 128 * len(arrays), 0      # 128: the .npy header
+    for i, n in enumerate(sizes):          # water-filling: the smallest arrays whole, the rest capped
+        left = len(sizes) - i
+        if n * left > budget:
+            cap = budget // left
+            break
+        budget -= n
+    else:
+        cap = sizes[-1]
+    os.makedirs(dump_dir, exist_ok=True)
+    for k, (name, a) in enumerate(arrays):
+        assert a.dtype in (np.float32, np.float64), name
+        if a.nbytes > cap:
+            pos = np.random.default_rng(DUMP_SAMPLE_SEED + k).choice(a.size, cap // a.itemsize, replace=False)
+            a = a[np.sort(pos)]
+        np.save(os.path.join(dump_dir, name + ".npy"), a)
+
+
 def time_region(torch, stream, fn, steps, after=None):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
@@ -481,9 +512,9 @@ def time_region(torch, stream, fn, steps, after=None):
     return e0.elapsed_time(e1) / steps
 
 
-def run_dense_single(mx, torch, stream, args, workload, steps, warmup, full):
+def run_dense_single(mx, torch, stream, args, workload, steps, warmup, full, dump_dir=None):
     """One dense workload on one GPU: parity, device-resident timing, and (full) the front-end
-    variants and the host-buffer arm."""
+    variants and the host-buffer arm. dump_dir: where the timed path's outputs go (dump_outputs)."""
     dev = torch.device("cuda", 0)
     shapes = WORKLOADS[workload]["shapes"]()
     sizes = [int(np.prod(s)) for s in shapes]
@@ -519,6 +550,8 @@ def run_dense_single(mx, torch, stream, args, workload, steps, warmup, full):
     ms_step = time_region(torch, stream, step, steps)
     launches = mx.base.kernel_launch_count()
     clocks = sampler.stop()
+    if dump_dir:
+        dump_outputs(dump_dir, {"weight_%03d" % k: o.asnumpy() for k, o in enumerate(outs)})
     # the timed region is exactly K launches of the dominant kernel back to back on this stream:
     # its average launch duration (incl. launch gaps) is the region's duration / K
     alg = algorithmic_bytes(workload, 1)
@@ -625,7 +658,8 @@ def run_single_gpu(args):
             sys.exit(3)
         return
 
-    main = run_dense_single(mx, torch, stream, args, args.workload, args.steps, args.warmup, full=True)
+    main = run_dense_single(mx, torch, stream, args, args.workload, args.steps, args.warmup, full=True,
+                            dump_dir=args.dump_outputs)
     configs = {}
     if not args.no_config_legs:
         other = "bert_adam" if args.workload == "resnet50_sgd" else "resnet50_sgd"
@@ -685,7 +719,16 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config-legs", action="store_true",
                     help="skip the short legs over the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned to DIR/*.npy (at most "
+                         "64 MB, longer outputs sampled): the pulled weights (dense workloads) or every "
+                         "puller's row ids and rows (rsp). One-GPU runs only: with --gpus > 1 each rank is "
+                         "a separate torchrun process, and that arm does not dump")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs covers --impl b200 on one GPU")
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
         # torchrun exports OMP_NUM_THREADS=1 to every rank; the CPU arm is entitled to all host

@@ -116,9 +116,10 @@ def _time(torch, stream, fn, steps, after):
     return e0.elapsed_time(e1) / steps
 
 
-def run_single_gpu_leg(mx, torch, stream, steps, nval=8, host_arm=False):
-    """nval values on ONE GPU (what BASELINE configs[4] looks like from the store's side when the
-    driver gives us one GPU): timing + roofline + bit-exact check of the pulled rows."""
+def run_single_gpu_leg(mx, torch, stream, steps, nval=8, host_arm=False, dump_dir=None):
+    """nval values on ONE GPU (what BASELINE configs[4] looks like from the store's side on a single
+    GPU): timing + roofline + bit-exact check of the pulled rows. dump_dir: where
+    the last timed pull's outputs go (bench.dump_outputs; row ids as float64, exact below 2**53)."""
     import kvoracle as K
     from bench import measured_peaks
     shape = (ROWS, ROW_LEN)
@@ -158,6 +159,13 @@ def run_single_gpu_leg(mx, torch, stream, steps, nval=8, host_arm=False):
     mx.base.reset_kernel_launch_count()
     pull_ms = _time(torch, stream, pull_fn, steps, mx.nd.waitall)
     launches_pull = mx.base.kernel_launch_count() / steps
+    if dump_dir:
+        from bench import dump_outputs
+        dumped = {}
+        for i, out in enumerate(outs):
+            dumped["pull_%d_ids" % i] = out.indices.asnumpy().astype(np.float64)
+            dumped["pull_%d_rows" % i] = out.data.asnumpy()
+        dump_outputs(dump_dir, dumped)
     pb, lb, union = alg_bytes(idx, pull)
     peaks, peak_src = measured_peaks()
     res = {"workload": "row_sparse push + row_sparse_pull, table (%d, %d) fp32, %d values x %d rows, "
@@ -207,7 +215,7 @@ def run_single_gpu_line(mx, torch, stream, args):
     from bench import config_block, ClockSampler
     sampler = ClockSampler(0)
     sampler.start()
-    leg = run_single_gpu_leg(mx, torch, stream, args.steps, host_arm=True)
+    leg = run_single_gpu_leg(mx, torch, stream, args.steps, host_arm=True, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     w = table_init()
     idx, val, _ = make_inputs(8)

@@ -62,7 +62,10 @@ class OracleOps(object):
 
     def _preloaded(self, ins, outs, p, stride, has_mom, mp):
         n = int(p['num_weights'])
-        lrs, wds = ins[n * stride], ins[n * stride + 1]
+        self._multi_sgd(ins, outs, p, stride, has_mom, mp, ins[n * stride], ins[n * stride + 1])
+
+    def _multi_sgd(self, ins, outs, p, stride, has_mom, mp, lrs, wds):
+        n = int(p['num_weights'])
         clip, rescale = self._clipv(p), self._s(p, 'rescale_grad', 1.0)
         momentum = self._s(p, 'momentum', 0.0) if has_mom else 0.0
         L = self.o.lib
@@ -91,6 +94,25 @@ class OracleOps(object):
 
     def _op_preloaded_multi_mp_sgd_mom_update(self, i, o, p):
         self._preloaded(i, o, p, 4, True, True)
+
+    def _op_multi_sgd_update(self, i, o, p):
+        self._multi_sgd(i, o, p, 2, False, False, _tuple(p['lrs']), _tuple(p['wds']))
+
+    def _op_multi_sgd_mom_update(self, i, o, p):
+        self._multi_sgd(i, o, p, 3, True, False, _tuple(p['lrs']), _tuple(p['wds']))
+
+    def _op_multi_mp_sgd_update(self, i, o, p):
+        self._multi_sgd(i, o, p, 3, False, True, _tuple(p['lrs']), _tuple(p['wds']))
+
+    def _op_multi_mp_sgd_mom_update(self, i, o, p):
+        self._multi_sgd(i, o, p, 4, True, True, _tuple(p['lrs']), _tuple(p['wds']))
+
+    def _op_adam_update(self, ins, outs, p):
+        w, g, mean, var = ins
+        c = self._adam_common(p)
+        self.o.lib.kvo_adam_update(w.size, K._ptr(outs[0]), K._ptr(mean), K._ptr(var), K._ptr(w), K._ptr(g),
+                                   c['clip'], self._s(p, 'rescale_grad', 1.0), c['beta1'], c['beta2'],
+                                   self._s(p, 'lr', None), self._s(p, 'wd', 0.0), c['eps'], 1)
 
     def _adam_common(self, p):
         return dict(beta1=self._s(p, 'beta1', K.f32(0.9)), beta2=self._s(p, 'beta2', K.f32(0.999)),

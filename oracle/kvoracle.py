@@ -33,6 +33,19 @@ def build(ref=True):
         subprocess.run(["make", "-s", "-C", _HERE, "ref"], check=True)
 
 
+def reference_tree():
+    """The reference's source tree: $B200KV_REFERENCE_TREE, else the tree oracle/_ref/libmxref.so was
+    built from (`make ref` records it); None when neither names a tree that exists here."""
+    t = os.environ.get("B200KV_REFERENCE_TREE")
+    if not t:
+        try:
+            with open(os.path.join(_HERE, "_ref", "reference_tree")) as f:
+                t = f.read().strip()
+        except OSError:
+            return None
+    return t if os.path.isdir(os.path.join(t, "src", "kvstore")) else None
+
+
 def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data)
 

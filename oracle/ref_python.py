@@ -32,12 +32,14 @@ import numpy as np
 
 import kvoracle as K
 
-REF_PY = "/root/reference/python/mxnet"
+_TREE = K.reference_tree()
+REF_PY = os.path.join(_TREE, "python", "mxnet") if _TREE else None
 
 
 def available():
     r = K.ref()
-    return os.path.isfile(os.path.join(REF_PY, "optimizer", "optimizer.py")) and r is not None and r.has_ops()
+    return REF_PY is not None and os.path.isfile(os.path.join(REF_PY, "optimizer", "optimizer.py")) and \
+        r is not None and r.has_ops()
 
 
 class Context(object):
@@ -88,7 +90,7 @@ class NDArray(object):
     def __mul__(self, scalar):
         # NDArray * python scalar -> _mul_scalar(scalar=str(scalar)): the scalar goes through dmlc::stof
         LOG.append(('_mul_scalar', {'scalar': str(scalar)}))
-        s = np.float32(K.ref().dmlc_stof(repr(float(scalar))))
+        s = np.float32(_stof(repr(float(scalar))))
         return NDArray((self.a * s).astype(self.a.dtype), self.context)
 
     def __iadd__(self, other):
@@ -123,6 +125,25 @@ def cast(data, dtype, out=None):
 
 LOG = []          # (operator, {parameter: string}) of every call, in order -- compared between front-ends
 
+# what runs the operators and parses scalar parameters: the reference's own code (oracle/_ref) unless
+# use_oracle_ops() switched to the plain-C restatement (golden_ops.OracleOps, kvoracle.dmlc_stof)
+_OPS = {}
+
+
+def use_oracle_ops(on=True):
+    _OPS.clear()
+    if on:
+        import golden_ops
+        _OPS.update(invoke=golden_ops.OracleOps().invoke, stof=K.dmlc_stof)
+
+
+def _op_invoke(*args, **params):
+    return (_OPS.get('invoke') or K.ref().op_invoke)(*args, **params)
+
+
+def _stof(text):
+    return (_OPS.get('stof') or K.ref().dmlc_stof)(text)
+
 
 def _flat(x):
     out = []
@@ -132,13 +153,17 @@ def _flat(x):
 
 
 def _invoke(name, args, out, kwargs, new_out=None):
-    ins = [a.a.reshape(-1) for a in _flat(args)]
+    views = {}
+
+    def view(a):                 # an array both read and written is one and the same view
+        return views.setdefault(id(a), a.a.reshape(-1))
+    ins = [view(a) for a in _flat(args)]
     params = {k: v for k, v in kwargs.items()}
     LOG.append((name, {k: str(v) for k, v in params.items()}))
     if out is None:
         out = new_out(ins, params)
     outs = _flat([out])
-    K.ref().op_invoke(name, ins, [o.a.reshape(-1) for o in outs], **params)
+    _op_invoke(name, ins, [view(o) for o in outs], **params)
     return out
 
 
@@ -254,7 +279,7 @@ def reference_python():
     """with reference_python() as (opt, sched): opt = the reference's optimizer module, sched = its
     lr_scheduler module. The stand-in `mxnet.*` entries live in sys.modules only inside the block
     (Updater.__call__ imports ..numpy lazily), so nothing else in the process ever sees them."""
-    assert available(), "needs /root/reference and oracle/_ref/libmxref.so"
+    assert available(), "needs the reference tree (kvoracle.reference_tree) and oracle/_ref/libmxref.so"
     saved = {k: v for k, v in sys.modules.items() if k == 'mxnet' or k.startswith('mxnet.')}
     for k in saved:
         del sys.modules[k]

@@ -171,8 +171,8 @@ def test_optimizer_record_rules(mx):
 
 
 # ---------------------------------------------------------------- drop-in boundary: signatures
-_REF_HEADERS = [("/root/reference/include/mxnet/c_api.h", "MXNET_DLL"),
-                ("/root/reference/3rdparty/tvm/nnvm/include/nnvm/c_api.h", "NNVM_DLL")]
+# headers of the reference's source tree, read only while its results are recorded (oracle/refrecord.py)
+_REF_HEADERS = [("include/mxnet/c_api.h", "MXNET_DLL"), ("3rdparty/tvm/nnvm/include/nnvm/c_api.h", "NNVM_DLL")]
 _BASE = {'int', 'char', 'void', 'float', 'double', 'size_t', 'bool', 'uint32_t', 'int64_t', 'uint64_t', 'unsigned',
          'const', 'int32_t', 'uint8_t'}
 
@@ -238,41 +238,45 @@ def _resolve(toks, typedefs):
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(_REF_HEADERS[0][0]), reason="needs /root/reference")
 def test_signatures_match_reference_headers():
     """every MX* / NN* function include/b200kv_c_api.h declares has, type for type, the signature the
     reference declares in include/mxnet/c_api.h (or nnvm/c_api.h): return type, parameter count, every
     parameter's type after resolving the handle typedefs -- so a binding written against the
     reference's header binds libb200kv.so unchanged"""
+    import refrecord as R
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     mine, my_td = _c_declarations(os.path.join(root, "include", "b200kv_c_api.h"), "B200KV_DLL")
-    ref, ref_td = {}, {}
-    for path, macro in _REF_HEADERS:
-        f, t = _c_declarations(path, macro)
-        ref.update(f)
-        ref_td.update(t)
-    checked = 0
-    for name, (ret, params) in sorted(mine.items()):
-        if name.startswith("B200KV"):
-            continue                           # extensions: no reference counterpart
-        assert name in ref, "%s is not a function of the reference's C API" % name
-        rret, rparams = ref[name]
-        assert _resolve(ret, my_td) == _resolve(rret, ref_td), name
-        assert len(params) == len(rparams), (name, params, rparams)
-        for i, (a, b) in enumerate(zip(params, rparams)):
-            assert _resolve(a, my_td) == _resolve(b, ref_td), (name, i, a, b)
-        checked += 1
-    assert checked >= 60
-    # the callback types those functions take
-    for cb in ("MXKVStoreUpdater", "MXKVStoreStrUpdater", "MXKVStoreServerController", "EngineAsyncFunc",
-               "EngineSyncFunc", "EngineFuncParamDeleter"):
-        assert my_td[cb][0].startswith('fn') and my_td[cb][0] == ref_td[cb][0], cb
-        assert _resolve(my_td[cb][1:], {k: v for k, v in my_td.items() if k != cb}) == \
-            _resolve(ref_td[cb][1:], {k: v for k, v in ref_td.items() if k != cb}), cb
+    names = sorted(n for n in mine if not n.startswith("B200KV"))     # B200KV*: extensions, no counterpart
+    callbacks = ("MXKVStoreUpdater", "MXKVStoreStrUpdater", "MXKVStoreServerController", "EngineAsyncFunc",
+                 "EngineSyncFunc", "EngineFuncParamDeleter")
+
+    def signatures(fns, td):
+        """function -> digest of (resolved return type, resolved parameter types)"""
+        out = {n: R.digest_json([_resolve(ret, td), [_resolve(a, td) for a in params]])
+               for n, (ret, params) in fns.items()}
+        for cb in callbacks:                   # the callback types those functions take
+            out[cb] = R.digest_json([td[cb][0], _resolve(td[cb][1:], {k: v for k, v in td.items() if k != cb})])
+        return out
+
+    def reference(_):
+        ref, ref_td = {}, {}
+        for path, macro in _REF_HEADERS:
+            f, t = _c_declarations(os.path.join(R.tree(), path), macro)
+            ref.update(f)
+            ref_td.update(t)
+        return signatures(ref, ref_td)
+    want = R.reference("test_abi::signatures", reference)
+    got = signatures(mine, my_td)
+    for name in names:
+        assert name in want, "%s is not a function of the reference's C API" % name
+        assert got[name] == want[name], "%s: return or parameter types differ from the reference's %s" % (
+            name, mine[name])
+    assert len(names) >= 60
+    for cb in callbacks:
+        assert my_td[cb][0].startswith('fn') and got[cb] == want[cb], "callback type %s differs: %s" % (
+            cb, my_td[cb])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/python/mxnet/kvstore/kvstore.py"),
-                    reason="needs /root/reference")
 def test_python_kvstore_surface_matches_reference():
     """boundary B1: every method / property of the reference's python KVStore and KVStoreBase classes
     (python/mxnet/kvstore/{kvstore,base}.py, parsed, not imported) exists on this package's classes
@@ -288,30 +292,36 @@ def test_python_kvstore_surface_matches_reference():
                         out[f.name] = ([a.arg for a in f.args.args], [ast.unparse(d) for d in f.args.defaults],
                                        [ast.unparse(d) for d in f.decorator_list])
         return out
+    import refrecord as R
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    files = (("kvstore.py", "KVStore"), ("base.py", "KVStoreBase"))
+    # the reference's methods: name -> digest of (parameter names, defaults, decorators)
+    want = R.reference("test_abi::python_kvstore_surface", lambda _: {
+        cls: {n: R.digest_json(sig) for n, sig in methods(os.path.join(R.tree(), "python/mxnet/kvstore", fname), cls).items()}
+        for fname, cls in files})
     total = 0
-    for fname, cls in (("kvstore.py", "KVStore"), ("base.py", "KVStoreBase")):
-        ref = methods("/root/reference/python/mxnet/kvstore/" + fname, cls)
+    for fname, cls in files:
         mine = methods(os.path.join(root, "anand_mxnet_b200", "kvstore", fname), cls)
-        assert len(ref) >= 10
-        for name, sig in ref.items():
+        assert len(want[cls]) >= 10
+        for name, sig in want[cls].items():
             assert name in mine, "%s.%s is missing" % (cls, name)
-            assert mine[name] == sig, (cls, name, mine[name], sig)
+            assert R.digest_json(list(mine[name])) == sig, \
+                "%s.%s: parameters, defaults or decorators differ from the reference's: %s" % (cls, name, mine[name])
             total += 1
     assert total >= 25
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/python/mxnet/kvstore/base.py"),
-                    reason="needs /root/reference")
 def test_key_value_marshalling_vs_reference(mx):
     """kvstore/base.py:_ctype_key_value here is a one-pass rewrite of the reference's recursive helper
     (python/mxnet/kvstore/base.py:33-65). The reference's function -- and the ctypes helpers it uses
     from python/mxnet/base.py -- are compiled from their source text at run time (ast; nothing is
     imported, libmxnet is not needed) and both are fed the same keys / values: same C key array, same
-    handle order, same str-key flag, same refusals."""
+    handle order, same str-key flag, same refusals. What the reference's function returned is stored
+    by oracle/refrecord.py, handles as their position in the list of arrays fed to it."""
     import ast
     import ctypes
     from array import array
+    import refrecord as R
     from anand_mxnet_b200.base import _LIB
     from anand_mxnet_b200.kvstore.base import _ctype_key_value as mine
     from anand_mxnet_b200.ndarray import NDArray
@@ -324,25 +334,29 @@ def test_key_value_marshalling_vs_reference(mx):
                     found[n.name] = n            # python-2 / python-3 twins: the later one is python 3's
         assert sorted(found) == sorted(names), (path, names)
         return ast.Module(body=sorted(found.values(), key=lambda n: n.lineno), type_ignores=[])
-    ns = {'ctypes': ctypes, 'array': array, 'NDArray': NDArray, 'string_types': (str,), 'py_str': lambda b: b.decode()}
-    exec(compile(functions("/root/reference/python/mxnet/base.py",
-                           ['c_str', 'c_str_array', 'c_array', 'c_array_buf', 'c_handle_array']),
-                 "reference base.py", "exec"), ns)
-    exec(compile(functions("/root/reference/python/mxnet/kvstore/base.py", ['_ctype_key_value']),
-                 "reference kvstore/base.py", "exec"), ns)
-    ref = ns['_ctype_key_value']
+
+    def reference_helper():
+        ns = {'ctypes': ctypes, 'array': array, 'NDArray': NDArray, 'string_types': (str,),
+              'py_str': lambda b: b.decode()}
+        exec(compile(functions(os.path.join(R.tree(), "python/mxnet/base.py"),
+                               ['c_str', 'c_str_array', 'c_array', 'c_array_buf', 'c_handle_array']),
+                     "reference base.py", "exec"), ns)
+        exec(compile(functions(os.path.join(R.tree(), "python/mxnet/kvstore/base.py"), ['_ctype_key_value']),
+                     "reference kvstore/base.py", "exec"), ns)
+        return ns['_ctype_key_value']
 
     def nd():
         h = ctypes.c_void_p()
         assert _LIB.MXNDArrayCreateNone(ctypes.byref(h)) == 0        # an empty handle: no device needed
         return NDArray(h)
     a = [nd() for _ in range(12)]
+    pos = {x.handle.value: i for i, x in enumerate(a)}
 
     def flat(res):
         keys, handles, use_str = res
         ks = [k.decode() if isinstance(k, bytes) else int(k) for k in keys]
         hs = [h if isinstance(h, int) else ctypes.cast(h, ctypes.c_void_p).value for h in handles]
-        return ks, hs, bool(use_str)
+        return [ks, [pos[h] for h in hs], bool(use_str)]
     cases = [
         (3, a[0]), ('w', a[0]), (3, [a[0], a[1], a[2]]), ('w', (a[0], a[1])),
         ([1, 2, 3], [a[0], a[1], a[2]]), (['a', 'b'], [a[0], a[1]]), ((5, 4), (a[0], a[1])),
@@ -353,12 +367,20 @@ def test_key_value_marshalling_vs_reference(mx):
         ([], []), ([4], [[]]),
         (list(range(157)), [[a[i % 12], a[(i + 1) % 12]] for i in range(157)]),
     ]
-    for keys, vals in cases:
-        assert flat(mine(keys, vals)) == flat(ref(keys, vals)), (keys,)
-    # what the reference refuses, this refuses
-    for keys, vals in [([1, 'a'], [a[0], a[1]]), ([1, 2], [a[0]]), (1.5, a[0]), ([1.5], [a[0]]),
-                       (['a', 2], [[a[0]], [a[1]]])]:
-        with pytest.raises(AssertionError):
-            ref(keys, vals)
-        with pytest.raises(AssertionError):
-            mine(keys, vals)
+    # and what the reference refuses
+    refused = [([1, 'a'], [a[0], a[1]]), ([1, 2], [a[0]]), (1.5, a[0]), ([1.5], [a[0]]),
+               (['a', 2], [[a[0]], [a[1]]])]
+
+    def run(fn):
+        def refuses(keys, vals):
+            try:
+                fn(keys, vals)
+            except AssertionError:
+                return True
+            return False
+        return [flat(fn(keys, vals)) for keys, vals in cases], [refuses(k, v) for k, v in refused]
+    want = R.reference("test_abi::ctype_key_value", lambda _: run(reference_helper()))
+    got = run(mine)
+    for i, (case, g, w) in enumerate(zip(cases, got[0], want[0])):
+        assert g == w, "case %d, keys %r: got %r, the reference returned %r" % (i, case[0], g, w)
+    assert want[1] == [True] * len(refused) and got[1] == want[1]

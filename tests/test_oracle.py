@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import kvoracle as K
+import refrecord as R
 
 
 def eq(a, b):
@@ -267,67 +268,64 @@ def test_rowsparse_reduce_retain_unique_golden(oracle, golden):
         assert np.array_equal(oracle.unique(ids), g["unique_%s" % tag]), tag
 
 
-# ---------------------------------------------------------------- live reference (when built here)
-needs_ref = pytest.mark.skipif(K.ref() is None, reason="oracle/_ref/libmxref.so not built")
-
-
-@needs_ref
+# ---------------------------------------------------------------- the reference's own code (stored results)
 def test_reduce_vs_reference_live(oracle):
-    r = K.ref()
     rng = np.random.default_rng(3)
-    for n in (1, 2, 3, 4, 5, 6, 7, 8, 9, 13, 16):
-        srcs = [rng.uniform(-1, 1, 3001).astype(np.float32) for _ in range(n)]
-        assert eq(oracle.reduce(srcs, "local"), r.reduce(srcs)), n
+    cases = [([rng.uniform(-1, 1, 3001).astype(np.float32) for _ in range(n)], 1)
+             for n in (1, 2, 3, 4, 5, 6, 7, 8, 9, 13, 16)]
     # above MXNET_KVSTORE_BIGARRAY_BOUND: 4 threads x 4096-element tasks (comm.h:394-410)
-    srcs = [rng.uniform(-1, 1, 1200007).astype(np.float32) for _ in range(8)]
-    assert eq(oracle.reduce(srcs, "local", nthreads=4), r.reduce(srcs, nthreads=4))
+    cases.append(([rng.uniform(-1, 1, 1200007).astype(np.float32) for _ in range(8)], 4))
+    want = R.reference("test_oracle::reduce", lambda r: [R.digest(r.reduce(s, nthreads=t)) for s, t in cases])
+    for i, ((s, t), w) in enumerate(zip(cases, want)):
+        assert R.digest(oracle.reduce(s, "local", nthreads=t)) == w, "%d sources of %d, %d threads" % (
+            len(s), s[0].size, t)
 
 
-@needs_ref
 def test_dmlc_stof_vs_reference_live():
     import random
-    r = K.ref()
     random.seed(7)
-    for _ in range(5000):
-        v = random.choice([random.uniform(0, 2), 10 ** random.uniform(-12, 6),
-                           0.1 * 0.97 ** random.randint(0, 500), -random.uniform(0, 1e-3)])
-        assert np.float32(K.dmlc_stof(repr(v))) == np.float32(r.dmlc_stof(repr(v))), v
+    texts = [repr(random.choice([random.uniform(0, 2), 10 ** random.uniform(-12, 6),
+                                 0.1 * 0.97 ** random.randint(0, 500), -random.uniform(0, 1e-3)]))
+             for _ in range(5000)]
+    want = R.reference("test_oracle::dmlc_stof",
+                       lambda r: R.digest(np.float32([r.dmlc_stof(t) for t in texts])))
+    assert R.digest(np.float32([K.dmlc_stof(t) for t in texts])) == want
 
 
-@needs_ref
 @pytest.mark.parametrize("clip", (None, 0.5, 0.002))
 def test_optimizers_vs_reference_live(oracle, clip):
-    r = K.ref()
     rng = np.random.default_rng(4)
     n = 10007
-
-    def mk():
-        return [rng.uniform(-1, 1, n).astype(np.float32) for _ in range(4)]
-    w, g, m, v = mk()
-    assert eq(oracle.sgd_update(w.copy(), g, .1, 1e-4, 1 / 256, clip),
-              r.sgd_update(w.copy(), g, .1, 1e-4, 1 / 256, clip))
-    a, b = [w.copy(), m.copy()], [w.copy(), m.copy()]
-    oracle.sgd_mom_update(a[0], g, a[1], .1, .9, 1e-4, 1 / 256, clip)
-    r.sgd_mom_update(b[0], g, b[1], .1, .9, 1e-4, 1 / 256, clip)
-    assert eq(a[0], b[0]) and eq(a[1], b[1])
-    a, b = [w.copy(), m.copy()], [w.copy(), m.copy()]
-    oracle.multi_sgd_update(a[0], g, a[1], .1, .9, 1e-4, 1 / 256, clip)
-    r.multi_sgd_update([b[0]], [g], [b[1]], [.1], [1e-4], .9, 1 / 256, clip)
-    assert eq(a[0], b[0]) and eq(a[1], b[1])
+    w, g, m, v = [rng.uniform(-1, 1, n).astype(np.float32) for _ in range(4)]
     v = np.abs(v)
-    a, b = [w.copy(), m.copy(), v.copy()], [w.copy(), m.copy(), v.copy()]
-    oracle.adam_update(a[0], g, a[1], a[2], 1e-3, wd=.01, clip=clip)
-    r.adam_update(b[0], g, b[1], b[2], 1e-3, wd=.01, clip=clip)
-    assert all(eq(x, y) for x, y in zip(a, b))
+
+    def run(sgd, sgd_mom, multi_sgd, adam):
+        out = [sgd(w.copy(), g, .1, 1e-4, 1 / 256, clip)]
+        b = [w.copy(), m.copy()]
+        sgd_mom(b[0], g, b[1], .1, .9, 1e-4, 1 / 256, clip)
+        out += b
+        b = [w.copy(), m.copy()]
+        multi_sgd(b[0], g, b[1])
+        out += b
+        b = [w.copy(), m.copy(), v.copy()]
+        adam(b[0], g, b[1], b[2], 1e-3, wd=.01, clip=clip)
+        return dict(zip(('sgd_w', 'sgd_mom_w', 'sgd_mom_mom', 'multi_sgd_w', 'multi_sgd_mom', 'adam_w',
+                         'adam_mean', 'adam_var'), [R.digest(x) for x in out + b]))
+    want = R.reference("test_oracle::optimizers[%s]" % clip, lambda r: run(
+        r.sgd_update, r.sgd_mom_update,
+        lambda w_, g_, m_: r.multi_sgd_update([w_], [g_], [m_], [.1], [1e-4], .9, 1 / 256, clip),
+        r.adam_update))
+    got = run(oracle.sgd_update, oracle.sgd_mom_update,
+              lambda w_, g_, m_: oracle.multi_sgd_update(w_, g_, m_, .1, .9, 1e-4, 1 / 256, clip),
+              oracle.adam_update)
+    for name in want:
+        assert got[name] == want[name], name
 
 
-@needs_ref
 def test_rowsparse_reduce_retain_vs_reference_live(oracle):
     """random layouts against the reference's own code (oracle/ref_sparse.cc), any thread count"""
-    r = K.ref()
-    if not r.has_sparse():
-        pytest.skip("oracle/_ref/libmxref.so predates ref_sparse.cc")
     rng = np.random.default_rng(11)
+    trials = []
     for trial in range(60):
         rows, rl = int(rng.integers(1, 400)), int(rng.integers(1, 70))
         nsrc = int(rng.integers(1, 10))
@@ -336,24 +334,32 @@ def test_rowsparse_reduce_retain_vs_reference_live(oracle):
             c = int(rng.integers(0, rows + 1)) if rng.random() < 0.8 else 0
             idxs.append(np.sort(rng.choice(rows, c, replace=False)).astype(np.int64))
             vals.append(rng.uniform(-1, 1, (c, rl)).astype(np.float32))
-        oi, ov = oracle.rsp_reduce(idxs, vals)
-        ri, rv = r.rsp_reduce(idxs, vals, nthreads=int(rng.integers(1, 6)))
-        assert np.array_equal(oi, ri) and eq(ov, rv), trial
+        nthreads = int(rng.integers(1, 6))
         ids = rng.integers(0, rows, int(rng.integers(0, 2 * rows + 1))).astype(np.int64)
-        assert np.array_equal(oracle.unique(ids), r.unique(ids)), trial
-        for req in (ids, oracle.unique(ids)):
-            a = oracle.sparse_retain(oi, ov, req)
-            b = r.sparse_retain(oi, ov, req)
-            assert np.array_equal(a[0], b[0]) and eq(a[1], b[1]), trial
-        # ascending unique ids: the reference's row-block kernel is the third witness
-        req = oracle.unique(ids)
-        b = r.sparse_retain(oi, ov, req, row_block=True)
-        a = oracle.sparse_retain(oi, ov, req)
-        assert np.array_equal(a[0], b[0]) and eq(a[1], b[1]), trial
         dense = rng.uniform(-1, 1, (rows, rl)).astype(np.float32)
-        a = oracle.sparse_retain(np.arange(rows), dense, ids, src_dense_rows=True)
-        b = r.sparse_retain(np.arange(rows), dense, ids, src_dense_rows=True)
-        assert np.array_equal(a[0], b[0]) and eq(a[1], b[1]), trial
+        trials.append((rows, idxs, vals, nthreads, ids, dense))
+
+    def run(rsp_reduce, unique, retain, retain_row_block):
+        out = []
+        for rows, idxs, vals, nthreads, ids, dense in trials:
+            ri, rv = rsp_reduce(idxs, vals, nthreads)
+            u = unique(ids)
+            res = [(ri, rv), (u, None)] + [retain(ri, rv, req) for req in (ids, u)]
+            res.append(retain_row_block(ri, rv, u))
+            res.append(retain(np.arange(rows), dense, ids, src_dense_rows=True))
+            out.append([[R.digest(np.asarray(a, np.int64)), None if b is None else R.digest(b)]
+                        for a, b in res])
+        return out
+    # ascending unique ids: the reference's row-block retain kernel is a third witness
+    want = R.reference("test_oracle::rowsparse_reduce_retain", lambda r: run(
+        lambda i, v, t: r.rsp_reduce(i, v, nthreads=t), r.unique, r.sparse_retain,
+        lambda i, v, q: r.sparse_retain(i, v, q, row_block=True)))
+    got = run(lambda i, v, t: oracle.rsp_reduce(i, v), oracle.unique, oracle.sparse_retain,
+              oracle.sparse_retain)
+    steps = ('reduce', 'unique', 'retain', 'retain unique ids', 'retain row-block', 'retain dense rows')
+    for trial, (g, w) in enumerate(zip(got, want)):
+        for step, a, b in zip(steps, g, w):
+            assert a == b, "trial %d: %s (ids, values) differ" % (trial, step)
 
 
 def _key_lists(rng, trials):
@@ -392,27 +398,25 @@ def test_group_order_small_calls_and_hook(oracle):
             assert list(pos) == want, (order, keys.size)
 
 
-@needs_ref
 def test_group_order_vs_reference_live(oracle):
     """the reference's own GroupKVPairs compiled against libstdc++ (oracle/ref_sparse.cc): equal to
     the restated order for every call; equal to CALL order up to 16 pairs; beyond that the values of a
     key are handed to the reduce in an order only std::sort's internals explain -- the finding
     DESIGN.md section 6 records, and what B200KV_GROUP_ORDER=reference reproduces."""
-    r = K.ref()
-    if not hasattr(r.lib, 'mxref_group_kv_pairs'):
-        pytest.skip("oracle/_ref/libmxref.so predates the grouping harness")
     rng = np.random.default_rng(22)
+    # last: the shape that matters, a list of keys with one value per device (10 keys x 4 GPUs)
+    calls = list(_key_lists(rng, 1500)) + [np.repeat(np.arange(10), 4)]
+    restated = [list(K.group_positions(k, 'reference')) for k in calls]
+    want = R.reference("test_oracle::group_order",
+                       lambda r: R.digest_json([list(r.group_positions(k)) for k in calls]))
+    assert R.digest_json(restated) == want                     # every call, position for position
     left_call_order = 0
-    for keys in _key_lists(rng, 1500):
-        live = r.group_positions(keys)
-        assert live == K.group_positions(keys, 'reference')
-        stable = K.group_positions(keys, 'call')
+    for keys, live in zip(calls, restated):
+        stable = list(K.group_positions(keys, 'call'))
         assert live[0] == stable[0]
         assert [sorted(g) for g in live[1]] == stable[1]          # same members, possibly another order
         if len(keys) <= 16:
             assert live == stable
         left_call_order += int(live != stable)
     assert left_call_order > 0
-    # the shape that matters: a list of keys with one value per device, e.g. 10 keys x 4 GPUs
-    keys = np.repeat(np.arange(10), 4)
-    assert r.group_positions(keys) != K.group_positions(keys, 'call')
+    assert restated[-1] != list(K.group_positions(calls[-1], 'call'))

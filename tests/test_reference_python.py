@@ -12,15 +12,21 @@ precision states, LARS's layer split and LAMB's step counts are all the referenc
     Python cannot travel to the GPU box, the fixture does) -- checked here against the model, and
     against the CUDA store in tests/test_updater_reference_fixture_gpu.py.
 
-The live halves need /root/reference and are skipped where it is absent (the GPU box)."""
+What the reference front-end returned in each comparison -- num_update, its operator calls with their
+parameter strings, the weight and state arrays, the learning rates its schedulers gave -- is stored by
+oracle/refrecord.py, and the mirror runs over the plain-C operators (golden_ops.OracleOps) and
+schedulers that replay those learning rates, so these comparisons need neither the reference tree nor
+oracle/_ref. Checks that need a live object of the reference's classes (the fixture recomputed from the
+reference, FusedOptimizer records taken from a reference optimizer) are skipped where it is absent."""
 import numpy as np
 import pytest
 
 import kvoracle as K
 import ref_python as RP
+import refrecord as R
 from gen_golden import updater_cases, run_updater_case
 
-live = pytest.mark.skipif(not RP.available(), reason="needs /root/reference and oracle/_ref/libmxref.so")
+live = pytest.mark.skipif(not RP.available(), reason="needs the reference tree and oracle/_ref/libmxref.so")
 
 
 def eq(a, b):
@@ -66,8 +72,10 @@ def test_golden_trajectories_are_the_live_reference(golden, name):
 # ---------------------------------------------------------------- the tests/compat mirror
 def _mirror():
     """tests/compat/mxnet_optimizer.py with its operator imports replaced by the harness's, so it
-    runs on the same numpy buffers and the same reference operators as the reference front-end"""
+    runs on the same numpy buffers as the reference front-end, over the plain-C operators that
+    tests/test_oracle_ops.py pins bit for bit to the reference's own"""
     from compat import mxnet_optimizer as M
+    RP.use_oracle_ops()
     saved = dict(M.__dict__)
     M.__dict__.update(RP.op_table())
     M._contrib = type('contrib', (), {'multi_lamb_update': staticmethod(RP.multi_lamb_update),
@@ -162,6 +170,72 @@ def _with_mults(opt):
     return opt
 
 
+SCHEDULERS = ('FactorScheduler', 'MultiFactorScheduler', 'CosineScheduler', 'PolyScheduler')
+SCHEDULE_LEN = 64          # num_update 0..63: beyond every plan below
+
+
+class _Recorder(object):
+    """stand-in lr_scheduler module over the reference's: keeps every scheduler it makes"""
+
+    def __init__(self, sched):
+        self.made = []
+        for name in SCHEDULERS:
+            setattr(self, name, self._maker(getattr(sched, name)))
+
+    def _maker(self, cls):
+        def make(**kw):
+            self.made.append(cls(**kw))
+            return self.made[-1]
+        return make
+
+
+def _schedules(name, build):
+    """[base_lr, learning rates for num_update 0..SCHEDULE_LEN-1 asked in increasing order as the
+    optimizers do] of each reference scheduler build(opt, sched) returns"""
+    def reference(_):
+        with RP.reference_python() as (opt, sched):
+            return [[s.base_lr, [s(n) for n in range(SCHEDULE_LEN)]] for s in build(opt, sched)]
+    return R.reference("test_reference_python::schedule[%s]" % name, reference)
+
+
+def _config_schedule(cfg):
+    def build(opt, sched):
+        rec = _Recorder(sched)
+        CONFIGS[cfg](opt, rec)          # the optimizer may set the scheduler's base_lr
+        return rec.made
+    return _schedules(cfg, build)
+
+
+class ReplayScheduler(object):
+    """a scheduler returning the learning rates a reference scheduler gave (_schedules), one table
+    per base_lr"""
+
+    def __init__(self, tables, base_lr):
+        self.tables = {b: r for b, r in tables}
+        self.base_lr = base_lr
+
+    @property
+    def base_lr(self):
+        return self._base
+
+    @base_lr.setter
+    def base_lr(self, v):
+        assert v in self.tables, "no learning rates recorded for base_lr %r" % v
+        self._base = v
+
+    def __call__(self, num_update):
+        return self.tables[self._base][num_update]
+
+
+class _Replay(object):
+    """stand-in lr_scheduler module for the mirror: its schedulers replay the recorded tables"""
+
+    def __init__(self, tables):
+        for name in SCHEDULERS:
+            setattr(self, name, lambda base_lr=tables[0][0] if tables else None, **kw:
+                    ReplayScheduler(tables, base_lr))
+
+
 def _norm(call):
     """(operator, parameters) with tuple-valued parameters as token lists: the mirror hands python
     tuples to the operators where the reference hands lists -- '(0.1,)' and '[0.1]' are the same
@@ -185,41 +259,50 @@ def _compare(cfg, mode, dtype=np.float32, steps=5, monkeypatch=None, agg=None, m
             o.multi_precision = True
             return o
     w0, grads = _plan(np.random.default_rng(len(cfg) + steps), steps, dtype)
-    with RP.reference_python() as (opt, sched):
-        want = _drive(opt, sched, make, w0, grads, mode, **kw)
-        M, saved = _mirror()
-        try:
-            got = _drive(M, sched, make, w0, grads, mode, **kw)
-        finally:
-            M.__dict__.clear()
-            M.__dict__.update(saved)
-    assert got[3] == want[3]                                  # num_update
-    assert len(got[2]) == len(want[2]) and len(want[2]) > 0
-    for a, b in zip(got[2], want[2]):                         # operator, parameter strings, order
-        assert _norm(a) == _norm(b)
-    for dev_g, dev_w in zip(got[0], want[0]):
+
+    def summary(res):
+        """weights and states as digests, every operator call as (operator, parameter tokens)"""
+        ws, states, log, num_update = res
+        return {'num_update': num_update,
+                'calls': [R.digest_json(list(_norm(c))) for c in log],
+                'weights': [[R.digest(w) for w in dev] for dev in ws],
+                'states': {'%d,%d' % key: [R.digest(a) for a in v] for key, v in sorted(states.items())}}
+
+    def reference(_):
+        with RP.reference_python() as (opt, sched):
+            return summary(_drive(opt, sched, make, w0, grads, mode, **kw))
+    key = "test_reference_python::%s|%s|%s|steps=%d|agg=%s|mp=%s|%s" % (
+        cfg, mode, np.dtype(dtype).name, steps, agg, mp, sorted(kw.items()))
+    want = R.reference(key, reference)
+    M, saved = _mirror()
+    try:
+        got = summary(_drive(M, _Replay(_config_schedule(cfg)), make, w0, grads, mode, **kw))
+    finally:
+        RP.use_oracle_ops(False)
+        M.__dict__.clear()
+        M.__dict__.update(saved)
+    assert got['num_update'] == want['num_update']
+    assert len(got['calls']) == len(want['calls']) and len(want['calls']) > 0
+    for i, (a, b) in enumerate(zip(got['calls'], want['calls'])):   # operator, parameter strings, order
+        assert a == b, (cfg, mode, 'operator call %d differs: the mirror called %r' % (i, RP.LOG[i]))
+    for d, (dev_g, dev_w) in enumerate(zip(got['weights'], want['weights'])):
         for k, (a, b) in enumerate(zip(dev_g, dev_w)):
-            assert eq(a, b), (cfg, mode, k)
-    assert got[1].keys() == want[1].keys()
-    for key in want[1]:
-        assert len(got[1][key]) == len(want[1][key])
-        for a, b in zip(got[1][key], want[1][key]):
-            assert eq(a, b), (cfg, mode, key)
+            assert a == b, (cfg, mode, 'device %d weight %d (%s) differs' % (d, k, NAMES[k]))
+    assert sorted(got['states']) == sorted(want['states']), (cfg, mode)
+    for st in want['states']:
+        assert got['states'][st] == want['states'][st], (cfg, mode, 'state (device, key) = ' + st)
 
 
-@live
 @pytest.mark.parametrize("mode", ['single', 'list'])
 @pytest.mark.parametrize("cfg", sorted(c for c in CONFIGS if c != 'test'))
 def test_compat_mirror_vs_reference(cfg, mode):
     _compare(cfg, mode)
 
 
-@live
 def test_compat_mirror_test_optimizer():
     _compare('test', 'single')
 
 
-@live
 @pytest.mark.parametrize("cfg", ['sgd_mom', 'sgd_plain_clip', 'lars', 'lars_no_momentum', 'lamb', 'adam'])
 @pytest.mark.parametrize("agg", [1, 3, 45])
 def test_compat_mirror_aggregation_sizes(cfg, agg, monkeypatch):
@@ -228,86 +311,118 @@ def test_compat_mirror_aggregation_sizes(cfg, agg, monkeypatch):
     _compare(cfg, 'list', monkeypatch=monkeypatch, agg=agg)
 
 
-@live
 @pytest.mark.parametrize("cfg", ['sgd_mom', 'sgd_plain_clip', 'lars', 'lars_no_momentum', 'lamb', 'adam'])
 @pytest.mark.parametrize("mode", ['single', 'list'])
 def test_compat_mirror_multi_precision_fp16(cfg, mode):
     _compare(cfg, mode, dtype=np.float16, mp=True)
 
 
-@live
 @pytest.mark.parametrize("cfg", ['sgd_mom', 'adam', 'lars_sched_correction', 'sgd_factor_sched'])
 def test_compat_mirror_shared_optimizer_two_devices(cfg):
     _compare(cfg, 'list', devices=2)
 
 
-@live
 @pytest.mark.parametrize("cfg", ['sgd_mom', 'adam', 'lamb'])
 def test_compat_mirror_set_learning_rate_between_steps(cfg):
     _compare(cfg, 'single', lr_changes={2: 0.01, 4: 0.3})
 
 
-@live
 @pytest.mark.parametrize("cfg", ['sgd_mom', 'adam', 'sgd_factor_sched'])
 def test_compat_mirror_state_pickle_restart(cfg):
     _compare(cfg, 'list', restart_at=3)
 
 
 # ---------------------------------------------------------------- the product's hyper-parameter record
-@live
+class _Param(object):
+    def __init__(self, lr_mult, wd_mult):
+        self.lr_mult, self.wd_mult = lr_mult, wd_mult
+
+
+_VARIANTS = [
+    dict(),
+    dict(param_idx2name=dict(enumerate(NAMES))),
+    dict(param_idx2name=dict(enumerate(NAMES)), param_dict={2: _Param(0.3, 0.7), 4: _Param(5.0, 0.0)}),
+    dict(param_dict={0: _Param(0.5, 2.0)}),
+]
+_SETTERS = [
+    ({}, {}),
+    ({1: 0.5, 'fc_weight': 2.0, 6: 0.25}, {0: 0.0, 'bn0_beta': 0.5, 'fc_bias': 3.0}),
+    ({'conv0_weight': 0.1, 0: 0.2}, {'emb_weight': 0.0}),          # index beats name
+]
+_INDICES = list(range(len(NAMES) + 2)) + ['fc_weight']
+_NUM_UPDATES = (0, 1, 3, 4, 7, 20)
+
+
+def _sched_variants(sched):
+    return [lambda: dict(lr_scheduler=sched.FactorScheduler(step=3, factor=0.5, base_lr=0.4)),
+            lambda: dict(lr_scheduler=sched.FactorScheduler(step=3, factor=0.5, base_lr=0.4), learning_rate=0.8),
+            lambda: dict(learning_rate=0.25), lambda: dict()]
+
+
+def _optimizers(mod):
+    """(class, variant, setter, optimizer) with lr = wd = 1, so _get_lr / _get_wd are the multipliers"""
+    for cls in ('SGD', 'Adam', 'Test'):
+        for v, kw in enumerate(_VARIANTS):
+            for t, (lr_mult, wd_mult) in enumerate(_SETTERS):
+                o = getattr(mod, cls)(learning_rate=1.0, wd=1.0, **kw)
+                o.set_lr_mult(lr_mult)
+                o.set_wd_mult(wd_mult)
+                yield cls, v, t, o
+
+
+def _learning_rates(o):
+    """learning_rate at each of _NUM_UPDATES, then whether set_learning_rate(0.03) is refused"""
+    rates = []
+    for n in _NUM_UPDATES:
+        o.num_update = n
+        rates.append(o.learning_rate)
+    try:
+        o.set_learning_rate(0.03)
+    except UserWarning:
+        return rates, True
+    assert o.learning_rate == 0.03
+    return rates, False
+
+
 def test_fused_record_vs_reference_optimizer():
     """anand_mxnet_b200.optimizer.FusedOptimizer (what kv.set_optimizer turns into the native replay's
     inputs) against the reference's Optimizer: multiplier lookup order (Parameter object, index, name),
-    default wd_mult of non-weights, scheduler / explicit learning rate precedence -- for records built
-    directly and for records taken from an object of the reference's own classes (record_of)."""
+    default wd_mult of non-weights, scheduler / explicit learning rate precedence -- the reference's
+    answers stored by oracle/refrecord.py"""
     from anand_mxnet_b200 import optimizer as P
 
-    class Param(object):
-        def __init__(self, lr_mult, wd_mult):
-            self.lr_mult, self.wd_mult = lr_mult, wd_mult
-    idx2name = dict(enumerate(NAMES))
-    variants = [
-        dict(),
-        dict(param_idx2name=idx2name),
-        dict(param_idx2name=idx2name, param_dict={2: Param(0.3, 0.7), 4: Param(5.0, 0.0)}),
-        dict(param_dict={0: Param(0.5, 2.0)}),
-    ]
-    setters = [
-        ({}, {}),
-        ({1: 0.5, 'fc_weight': 2.0, 6: 0.25}, {0: 0.0, 'bn0_beta': 0.5, 'fc_bias': 3.0}),
-        ({'conv0_weight': 0.1, 0: 0.2}, {'emb_weight': 0.0}),          # index beats name
-    ]
+    def reference(_):
+        with RP.reference_python() as (opt, sched):
+            mults = [[[o._get_lr(i), o._get_wd(i)] for i in _INDICES] for _, _, _, o in _optimizers(opt)]
+            rates = [_learning_rates(opt.SGD(**mk())) for mk in _sched_variants(sched)]
+            return {'multipliers': mults, 'learning_rates': rates}
+    want = R.reference("test_reference_python::fused_record", reference)
+    for (cls, v, t, mine), w in zip(_optimizers(P), want['multipliers']):
+        for i, m in zip(_INDICES, w):
+            assert list(mine.multipliers(i)) == m, (cls, sorted(_VARIANTS[v]), t, i)
+    tables = _schedules('fused_record', lambda opt, sched: [
+        sched.FactorScheduler(step=3, factor=0.5, base_lr=b) for b in (0.4, 0.8)])
+    for k, (mk, w) in enumerate(zip(_sched_variants(_Replay(tables)), want['learning_rates'])):
+        rates, refused = _learning_rates(P.SGD(**mk()))
+        assert [rates, refused] == w, k
+
+
+@live
+def test_record_of_reference_optimizer():
+    """FusedOptimizer records taken from objects of the reference's own optimizer classes (record_of):
+    the same multipliers, learning rates and operator parameters as the reference object"""
+    from anand_mxnet_b200 import optimizer as P
     with RP.reference_python() as (opt, sched):
-        for cls in ('SGD', 'Adam', 'Test'):
-            for kw in variants:
-                for lr_mult, wd_mult in setters:
-                    ref = getattr(opt, cls)(learning_rate=1.0, wd=1.0, **kw)
-                    mine = getattr(P, cls)(learning_rate=1.0, wd=1.0, **kw)
-                    for o in (ref, mine):
-                        o.set_lr_mult(lr_mult)
-                        o.set_wd_mult(wd_mult)
-                    assert P.fused_kind(ref) == cls.lower()
-                    rec = P.record_of(ref)
-                    for i in list(range(len(NAMES) + 2)) + ['fc_weight']:
-                        want = (ref._get_lr(i), ref._get_wd(i))       # lr = wd = 1: the multipliers
-                        assert mine.multipliers(i) == want, (cls, kw.keys(), i)
-                        assert rec.multipliers(i) == want, (cls, kw.keys(), i)
-        # learning rate: scheduler(num_update), an explicit rate overriding the scheduler's base
-        for mk in (lambda m: dict(lr_scheduler=sched.FactorScheduler(step=3, factor=0.5, base_lr=0.4)),
-                   lambda m: dict(lr_scheduler=sched.FactorScheduler(step=3, factor=0.5, base_lr=0.4),
-                                  learning_rate=0.8),
-                   lambda m: dict(learning_rate=0.25), lambda m: dict()):
-            ref, mine = opt.SGD(**mk(0)), P.SGD(**mk(0))
-            for n in (0, 1, 3, 4, 7, 20):
-                ref.num_update = mine.num_update = n
-                assert ref.learning_rate == mine.learning_rate == P.record_of(ref).learning_rate
-            for o in (ref, mine):
-                if o.lr_scheduler is None:
-                    o.set_learning_rate(0.03)
-                    assert o.learning_rate == 0.03
-                else:
-                    with pytest.raises(UserWarning):
-                        o.set_learning_rate(0.03)
+        for cls, v, t, ref in _optimizers(opt):
+            assert P.fused_kind(ref) == cls.lower()
+            rec = P.record_of(ref)
+            for i in _INDICES:
+                assert rec.multipliers(i) == (ref._get_lr(i), ref._get_wd(i)), (cls, v, t, i)
+        for mk in _sched_variants(sched):
+            ref = opt.SGD(**mk())
+            for n in _NUM_UPDATES:
+                ref.num_update = n
+                assert ref.learning_rate == P.record_of(ref).learning_rate
         # operator parameters handed to the library: the reference object's own attribute values
         ref = opt.Adam(learning_rate=2e-3, beta1=0.8, beta2=0.97, epsilon=1e-5, wd=0.1, rescale_grad=0.5,
                        clip_gradient=0.7, begin_num_update=11)
